@@ -1,7 +1,7 @@
 """bench.py — encoded docs/sec for GritLM-7B (random-init Mistral-7B weights), bf16, seq=512,
 batch=256 per GPU, through the B200-native encode path (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -10,7 +10,9 @@ final norm, masked-mean pool, L2 normalise) of one [256, 512] synthetic token ba
 Prints ONE JSON line (rank 0).  `value` = whole-job docs/s with inputs resident in HBM;
 `e2e` = the same through the host-buffer C-ABI call (H2D ids/mask + D2H embeddings in the timed
 region).  `--impl reference` times the reference algorithm (CPU oracle port of
-modeling_mistral_gritlm + GritLM.pooling) on the host cores on a bounded sample.
+modeling_mistral_gritlm + GritLM.pooling) on the host cores on a bounded sample.  `--dump-outputs DIR` writes the
+embeddings of the last timed step of both paths as DIR/<name>.npy (float32); the inputs are seeded, so two builds run
+with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -58,7 +60,32 @@ def parse():
     ap.add_argument("--config", type=int, default=1, choices=[1, 2, 3, 4],
                     help="BASELINE.json configs[] index: 1 = the headline encode line (default); 2 = in-batch contrastive "
                          "step, 3 = joint GRIT step, 4 = Mixtral-8x7B encode (scripts/other_configs.py)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the embeddings of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config != 1):
+        ap.error("--dump-outputs needs the B200 encode (--impl b200 --config 1)")
+    return args
+
+
+DUMP_BYTES = 60 << 20   # data bytes written by --dump-outputs; the .npy headers keep the files well inside 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each [rows, ...] array as out_dir/<name>.npy in float32.  When together they pass DUMP_BYTES, every array
+    keeps the same share of its rows, chosen by a fixed seed, so that two runs with the same arguments stay comparable."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = a.shape[0] * DUMP_BYTES // total
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(d / f"{name}.npy", a)
 
 
 def peaks():
@@ -326,10 +353,13 @@ def main():
     ids, mask = ids_host.to(dev), mask_host.to(dev)
     gathered = torch.empty(world * B, H, device=dev, dtype=torch.float32) if world > 1 else None
 
+    last = {}
+
     def step_device():
         emb = model.encode_pooled(ids, mask, None, "mean", True, is_causal=False)
         if world > 1:
             dist.all_gather_into_tensor(gathered, emb)  # every rank ends with all embeddings (SURVEY §8e)
+        last["emb"] = emb
         return emb
 
     host_step_ms = []
@@ -373,6 +403,9 @@ def main():
     n0 = lib.gritlm_b200_launch_count()
     ms_total = timed(step_device, K)
     launches = lib.gritlm_b200_launch_count() - n0
+    dumped = {}
+    if args.dump_outputs and rank == 0:   # what a caller of the timed path receives: all ranks' embeddings when gathered
+        dumped["embeddings"] = (gathered if world > 1 else last["emb"]).float().cpu().numpy()
     clocks = sampler.stop() if rank == 0 else None
     emb = step_device()
     ok = bool(torch.isfinite(emb).all()) and abs(emb.norm(dim=-1).mean().item() - 1.0) < 1e-3
@@ -384,6 +417,8 @@ def main():
         sampler2.start()
     ms_e2e = timed(step_host, K)
     clocks_e2e = sampler2.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # this rank's rows, written to the host buffer by the last timed call
+        dumped["embeddings_host"] = out_host.numpy().copy()
 
     # ---- the same K steps once more with the library's event profiler on: per-kernel durations INSIDE the step (sustained
     # clocks, warm L2 state of the real launch sequence) — kept out of the timed region above so that `value` carries no
@@ -549,6 +584,8 @@ def main():
                 line["cpu_baseline"] = {"value": v, "unit": UNIT, "cores": cores, "kind": "port", "sample": sample}
             except Exception as e:  # the GPU measurement above must survive a host-side failure (e.g. host memory)
                 line["cpu_baseline"] = {"value": None, "unit": UNIT, "kind": "port", "error": repr(e)[:200]}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -9,10 +9,9 @@ library.
 Parity pinning: the reference ships no tests or golden vectors (SURVEY.md §4), so this oracle is
 pinned against OUTPUTS OF THE REFERENCE ITSELF: `tests/golden/make_golden.py` imports the
 reference's own `scripts/modeling_mistral_gritlm.py`, `gritlm/gritlm.py` and
-`gritlm/training/model.py` (unmodified, from /root/reference) and stores their outputs on seeded
-inputs in `tests/golden/*.npz`; `tests/test_oracle_golden.py` checks this file against those
-fixtures, and `tests/test_oracle_vs_reference.py` re-runs the live comparison whenever
-/root/reference is present.
+`gritlm/training/model.py` (unmodified) and stores their outputs on seeded inputs in
+`tests/golden/*.npz`; `tests/test_oracle_golden.py` checks this file against those fixtures, and
+`tests/test_oracle_vs_reference.py` against a second set of inputs (`make_golden_checks.py`).
 """
 from __future__ import annotations
 

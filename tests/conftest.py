@@ -38,5 +38,9 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope="session")
 def golden():
+    """The Mistral fixture of tests/golden/make_golden.py, stored as three archives to keep each file small."""
     import numpy as np
-    return dict(np.load(ROOT / "tests" / "golden" / "gritlm_ref_tiny.npz"))
+    out = {}
+    for part in ("", "_eager", "_logits"):
+        out.update(np.load(ROOT / "tests" / "golden" / f"gritlm_ref_tiny{part}.npz"))
+    return out

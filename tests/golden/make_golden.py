@@ -1,7 +1,7 @@
-"""Generates tests/golden/gritlm_ref_tiny.npz by running the UNMODIFIED reference code from
-/root/reference on seeded inputs (run here, in the build container; the GPU box has no reference).
+"""Generates tests/golden/gritlm_ref_tiny.npz, gritlm_ref_tiny_eager.npz and gritlm_ref_tiny_logits.npz (one
+fixture, split so that each file stays small) by running the UNMODIFIED reference code on seeded inputs.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
 
 What is executed from the reference (imported, never copied):
   * scripts/modeling_mistral_gritlm.py  MistralModel / MistralForCausalLM  (sdpa + eager, is_causal True/False)
@@ -20,7 +20,7 @@ import numpy as np
 import torch
 
 ROOT = Path(__file__).resolve().parents[2]
-REF = Path("/root/reference")
+REF = None  # the reference checkout, from the command line
 sys.path.insert(0, str(ROOT))
 from oracle import gritlm_oracle as O  # noqa: E402
 
@@ -117,10 +117,14 @@ def main():
     for t in ("mixed", "token"):
         out[f"ntl_{t}"] = np.array([NextTokenLoss(dims.vocab_size, t, 0.5)(labels, logits).item()])
 
-    path = Path(__file__).with_name("gritlm_ref_tiny.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, f"{path.stat().st_size/1024:.0f} KiB", "keys:", len(out))
+    parts = {"_eager": [k for k in out if "_eager_" in k], "_logits": [k for k in out if k.startswith("logits_")]}
+    parts[""] = [k for k in out if not any(k in keys for keys in parts.values())]
+    for suffix, keys in parts.items():
+        path = Path(__file__).with_name(f"gritlm_ref_tiny{suffix}.npz")
+        np.savez_compressed(path, **{k: out[k] for k in keys})
+        print("wrote", path, f"{path.stat().st_size/1024:.0f} KiB", "keys:", len(keys))
 
 
 if __name__ == "__main__":
+    REF = Path(sys.argv[1]).resolve()
     main()

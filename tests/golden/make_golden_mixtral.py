@@ -1,7 +1,7 @@
 """Generates tests/golden/gritlm_ref_tiny_mixtral.npz by running the UNMODIFIED reference
-scripts/modeling_mixtral_gritlm.py (from /root/reference) on seeded inputs.
+scripts/modeling_mixtral_gritlm.py on seeded inputs.
 
-    python tests/golden/make_golden_mixtral.py
+    python tests/golden/make_golden_mixtral.py <reference checkout>
 
 Shims (SURVEY.md §8c): `transformers.utils.import_utils.is_torch_fx_available` (removed in
 transformers 5.x, used only for FX wrapping at mixtral:66-72) is stubbed to False before the file is
@@ -15,7 +15,7 @@ import numpy as np
 import torch
 
 ROOT = Path(__file__).resolve().parents[2]
-REF = Path("/root/reference")
+REF = None  # the reference checkout, from the command line
 sys.path.insert(0, str(ROOT))
 from oracle import gritlm_oracle as O  # noqa: E402
 
@@ -87,4 +87,5 @@ def main():
 
 
 if __name__ == "__main__":
+    REF = Path(sys.argv[1]).resolve()
     main()

@@ -10,6 +10,7 @@ import sys
 import time
 from pathlib import Path
 
+import numpy as np
 import pytest
 import torch
 
@@ -135,3 +136,39 @@ def test_gpu_arm_survives_a_failing_profiler(monkeypatch):
         lib.gritlm_b200_profile_read = lambda *a: 1     # the library reports an error
         line = run_main(monkeypatch, ["--batch", "2", "--layers", "2", "--steps", "1", "--warmup", "1", "--no-cpu-baseline"])
     assert line["value"] > 0 and "error" in line["roofline"]["in_step"]
+
+
+def test_dump_outputs_writes_the_timed_embeddings_the_same_every_run(monkeypatch, tmp_path):
+    runs = []
+    for i in range(2):
+        with cpu_stand_ins(monkeypatch, layers=2):
+            run_main(monkeypatch, ["--batch", "2", "--layers", "2", "--steps", "3", "--warmup", "1", "--no-cpu-baseline",
+                                   "--dump-outputs", str(tmp_path / str(i))])
+        runs.append({p.stem: np.load(p) for p in sorted((tmp_path / str(i)).iterdir())})
+    assert set(runs[0]) == {"embeddings", "embeddings_host"}
+    for name, a in runs[0].items():
+        assert a.dtype == np.float32 and a.shape == (2, H), name
+        np.testing.assert_allclose(np.linalg.norm(a, axis=-1), 1.0, rtol=1e-5)
+        np.testing.assert_array_equal(a, runs[1][name])      # seeded inputs: identical from run to run
+
+
+def test_dump_outputs_keeps_a_fixed_sample_of_rows_within_the_budget(monkeypatch, tmp_path):
+    sys.path.insert(0, str(ROOT))
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 64 * 16 * 4)
+    a = np.arange(100 * 16, dtype=np.float64).reshape(100, 16)
+    for d in ("x", "y"):
+        bench.dump_outputs(tmp_path / d, {"a": a, "b": a[:28]})
+    x, y = np.load(tmp_path / "x" / "a.npy"), np.load(tmp_path / "y" / "a.npy")
+    b = np.load(tmp_path / "x" / "b.npy")
+    assert x.dtype == b.dtype == np.float32 and x.nbytes + b.nbytes <= bench.DUMP_BYTES
+    assert len(x) == 50 and len(b) == 14 and np.array_equal(x, y)
+    assert np.array_equal(x, a[np.sort(x[:, 0].astype(int) // 16)])   # whole rows of the input, in order
+
+
+def test_steps_below_one_are_refused(monkeypatch):
+    sys.path.insert(0, str(ROOT))
+    import bench
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "0"])
+    with pytest.raises(SystemExit):
+        bench.parse()

@@ -1,24 +1,23 @@
-"""Live parity of the W3 training hooks: the UNMODIFIED reference `gritlm.training.model.GritLMTrainModel` and this
-repo's `gritlm_b200.training.GritLMTrainModel` run the same joint step (query + passages with instruction_lens,
-generative batch with labels) over the same random-init Mistral-shaped HF model on CPU and must return the same
-q_reps / p_reps / loss_emb / loss_gen / loss, and the same gradients at the representations.
+"""Parity of the W3 training hooks with the UNMODIFIED reference `gritlm.training.model.GritLMTrainModel`: both run the
+same joint step (query + passages with instruction_lens, generative batch with labels) over the same random-init
+Mistral-shaped HF model on CPU and must return the same q_reps / p_reps / loss_emb / loss_gen / loss, and the same
+gradients at the model parameters.  The reference's results are stored in tests/golden/train_model.npz
+(tests/golden/make_golden_checks.py runs the reference on `make_checkpoint` and `batch` below).
 
 The device calls are stand-ins (the HF module for the backbone, the oracle for the two loss kernels — each pinned to
 the reference separately in tests/test_oracle_vs_reference.py); what is compared is this repo's host logic of
 `GritLMTrainModel.encode / forward`, `DistributedContrastiveLoss` and the no-grad / precomputed-reps conventions
 (gritlm/training/model.py:112-222).  attn='cccc' so that the stock HF Mistral (no `is_causal` keyword) can stand in;
-the 'bb' flag is covered by tests/test_train_model_host_cpu.py.  Skipped where /root/reference is absent."""
-import sys
+the 'bb' flag is covered by tests/test_train_model_host_cpu.py."""
 from pathlib import Path
 
+import numpy as np
 import pytest
 import torch
 
 from oracle import gritlm_oracle as O
 
-REF = Path("/root/reference")
-pytestmark = pytest.mark.skipif(not (REF / "gritlm" / "training" / "model.py").exists(),
-                                reason="reference tree not present on this machine")
+GOLD = Path(__file__).parent / "golden" / "train_model.npz"
 TEMP, FACTOR = 0.05, 2.0
 
 
@@ -62,25 +61,37 @@ def oracle_kernel(q_all, p_all, temperature, q_row0, q_rows, p_row0, p_rows, nee
     return loss.detach(), (q.grad[q_row0:q_row0 + q_rows] if need_grad else None), (p.grad[p_row0:p_row0 + p_rows] if need_grad else None)
 
 
-@pytest.fixture(scope="module")
-def pair(tmp_path_factory):
+def make_checkpoint(d):
+    """The tiny random-init Mistral both sides load (seeded: the stored reference results depend on these weights)."""
     from transformers import MistralConfig, MistralForCausalLM
     cfg = MistralConfig(vocab_size=120, hidden_size=64, intermediate_size=96, num_hidden_layers=2, num_attention_heads=4,
                         num_key_value_heads=2, max_position_embeddings=128, sliding_window=None)
     torch.manual_seed(0)
-    d = tmp_path_factory.mktemp("mistral_tiny")
     MistralForCausalLM(cfg).float().save_pretrained(d)
-    sys.path.insert(0, str(REF))
-    from gritlm.training.model import GritLMTrainModel as RefTrainModel
-    ref = RefTrainModel(model_name_or_path=str(d), temperature=TEMP, negatives_cross_device=False, loss_gen_type="mixed",
-                        loss_gen_factor=FACTOR, pooling_method="mean", attn="cccc", normalized=True,
-                        torch_dtype=torch.float32)
+
+
+def weights_checksum(model):
+    return float(sum(p.detach().double().sum() for p in model.parameters()))
+
+
+@pytest.fixture(scope="module")
+def gold():
+    return dict(np.load(GOLD))
+
+
+@pytest.fixture(scope="module")
+def ours(tmp_path_factory, gold):
+    from transformers import AutoModelForCausalLM
+    d = tmp_path_factory.mktemp("mistral_tiny")
+    make_checkpoint(d)
+    hf = AutoModelForCausalLM.from_pretrained(str(d), dtype=torch.float32)     # as the reference loads it
+    assert weights_checksum(hf) == float(gold["weights_checksum"]), "the seeded checkpoint differs from the stored one"
     from gritlm_b200.training import DistributedContrastiveLoss, GritLMTrainModel
-    ours = GritLMTrainModel(model=HFLM(ref.model), device="cpu", attn="cccc", temperature=TEMP, loss_gen_type="mixed",
-                            loss_gen_factor=FACTOR, pooling_method="mean")
-    ours.emb_loss_fn = DistributedContrastiveLoss(TEMP, False, kernel=oracle_kernel)
-    ours.gen_loss_fn = lambda labels, logits: O.next_token_loss(labels, logits, 120, "mixed", FACTOR)
-    return ref, ours
+    model = GritLMTrainModel(model=HFLM(hf), device="cpu", attn="cccc", temperature=TEMP, loss_gen_type="mixed",
+                             loss_gen_factor=FACTOR, pooling_method="mean")
+    model.emb_loss_fn = DistributedContrastiveLoss(TEMP, False, kernel=oracle_kernel)
+    model.gen_loss_fn = lambda labels, logits: O.next_token_loss(labels, logits, 120, "mixed", FACTOR)
+    return model
 
 
 def batch(seed):
@@ -102,34 +113,33 @@ def clone(f):
     return {k: v.clone() for k, v in f.items()}
 
 
-def test_joint_step_outputs_match_reference(pair):
-    ref, ours = pair
+def near(x, name, gold, atol):
+    return torch.allclose(x, torch.from_numpy(gold[name]), atol=atol)
+
+
+def test_joint_step_outputs_match_reference(ours, gold):
     q, p, gen = batch(1)
-    a = ref(query=clone(q), passage=clone(p), generative=clone(gen))
     b = ours(query=clone(q), passage=clone(p), generative=clone(gen))
-    assert torch.allclose(b.q_reps, a.q_reps, atol=1e-6) and torch.allclose(b.p_reps, a.p_reps, atol=1e-6)
+    assert near(b.q_reps, "joint.q_reps", gold, 1e-6) and near(b.p_reps, "joint.p_reps", gold, 1e-6)
     for k in ("loss_emb", "loss_gen", "loss"):
-        assert abs(getattr(a, k).item() - getattr(b, k).item()) < 1e-5, k
-    # gradients w.r.t. the model parameters agree (same graph through the shared HF module)
-    params = [x for x in ref.model.parameters()]
-    ga = torch.autograd.grad(a.loss, params, allow_unused=True)
-    gb = torch.autograd.grad(b.loss, params, allow_unused=True)
-    for x, y in zip(ga, gb):
-        assert (x is None) == (y is None)
-        if x is not None:
-            assert torch.allclose(x, y, atol=1e-5, rtol=1e-4)
+        assert abs(float(gold[f"joint.{k}"]) - getattr(b, k).item()) < 1e-5, k
+    # gradients w.r.t. the model parameters agree (the reference's are stored by parameter name)
+    named = list(ours.model.hf.named_parameters())
+    grads = torch.autograd.grad(b.loss, [x for _, x in named], allow_unused=True)
+    unused = set(gold["joint.unused_params"].tolist())
+    for (name, _), y in zip(named, grads):
+        assert (name in unused) == (y is None), name
+        if y is not None:
+            assert torch.allclose(torch.from_numpy(gold[f"joint.grad.{name}"]), y, atol=1e-5, rtol=1e-4), name
 
 
-def test_embedding_only_no_grad_towers_and_precomputed_reps(pair):
-    ref, ours = pair
+def test_embedding_only_no_grad_towers_and_precomputed_reps(ours, gold):
     q, p, _ = batch(2)
-    a = ref(query=clone(q), passage=clone(p), q_grad=False)
     b = ours(query=clone(q), passage=clone(p), q_grad=False)
-    assert not b.q_reps.requires_grad and b.p_reps.requires_grad and a.loss_gen is None and b.loss_gen is None
-    assert abs(a.loss.item() - b.loss.item()) < 1e-5
+    assert not b.q_reps.requires_grad and b.p_reps.requires_grad and b.loss_gen is None
+    assert abs(float(gold["emb.loss"]) - b.loss.item()) < 1e-5
     # GradCache convention (gradcache_trainer.py:385-399): a positional dict is the query; cached reps bypass the encoder
-    a1, b1 = ref(clone(q)), ours(clone(q))
-    assert a1.p_reps is None and b1.p_reps is None and torch.allclose(a1.q_reps, b1.q_reps, atol=1e-6)
-    a2 = ref(q_reps=a.q_reps.detach(), p_reps=a.p_reps.detach())
-    b2 = ours(q_reps=a.q_reps.detach(), p_reps=a.p_reps.detach())
-    assert abs(a2.loss.item() - b2.loss.item()) < 1e-6
+    b1 = ours(clone(q))
+    assert b1.p_reps is None and near(b1.q_reps, "query_only.q_reps", gold, 1e-6)
+    b2 = ours(q_reps=torch.from_numpy(gold["emb.q_reps"]), p_reps=torch.from_numpy(gold["emb.p_reps"]))
+    assert abs(float(gold["cached.loss"]) - b2.loss.item()) < 1e-6
